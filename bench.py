@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                  # this repo's CUDA path, config 2 (one process per GPU)
     python bench.py --config star --steps K --warmup W             # config 3: 64 x 1280x960 semi-dense match_xfeat_star
     python bench.py --impl reference --steps K --warmup W          # the UNMODIFIED reference on the host CPU (oracle/_ref)
+    python bench.py --steps K --warmup W --dump-outputs DIR        # also write the last timed step's results as DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of 64 synthetic image pairs per GPU:
   sparse: detectAndCompute on both image sets (backbone, NMS/top-k 4096, bicubic descriptors) + per-pair MNN match;
@@ -290,6 +291,7 @@ def run_gpu(args):
     barrier()
     launches = lib.xfeat_launch_count() - launches0
     ms_total = t0.elapsed_time(t1)
+    dump = last_step_outputs(out, star) if args.dump_outputs and rank == 0 else None
     dom_ms = statistics.mean(a.elapsed_time(b) for a, b in dom_events)
 
     # ---- sustained self-check: the same resident step back to back for >= 2 s (clocks settle under the power cap) ----
@@ -414,9 +416,39 @@ def run_gpu(args):
                                         "sample": cpu_sample_text(c, args.config)}
             except Exception as e:   # reported, never silently dropped
                 line["cpu_baseline"] = {"value": None, "unit": "pairs/s", "cores": 0, "kind": "failed", "sample": str(e)[-300:]}
+        if dump is not None:
+            write_outputs(args.dump_outputs, dump)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+def last_step_outputs(out, star: bool):
+    """The arrays the timed step returns, as float32 / float64 host arrays.  Rows past a pair's count hold no result and are
+    zeroed, so two runs of the same build give identical files."""
+    import numpy as np
+
+    def valid_rows(x, n):
+        x = x.float().cpu().numpy()
+        x[np.arange(x.shape[1])[None, :] >= np.maximum(n, 0)[:, None]] = 0
+        return x
+
+    if star:
+        m, n_ref, cnt = out
+        n_ref = n_ref.cpu().numpy()
+        return {"matches": valid_rows(m, n_ref), "n_matches": n_ref.astype(np.float64),
+                "n_coarse_matches": cnt.cpu().numpy().astype(np.float64)}
+    mk0, mk1, cnt, n1, n2 = out
+    cnt = cnt.cpu().numpy()
+    return {"mkpts0": valid_rows(mk0, cnt), "mkpts1": valid_rows(mk1, cnt), "n_matches": cnt.astype(np.float64),
+            "n_keypoints0": n1.cpu().numpy().astype(np.float64), "n_keypoints1": n2.cpu().numpy().astype(np.float64)}
+
+
+def write_outputs(path: str, arrays: dict):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def main():
@@ -430,6 +462,9 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="sparse", choices=sorted(CONFIGS))
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0's batch) to DIR/<name>.npy; the inputs are seeded, "
+                         "so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -10,8 +10,6 @@ import torch
 
 pytestmark = pytest.mark.gpu
 
-from oracle import xfeat_oracle as orc  # noqa: E402
-
 
 @pytest.fixture(scope="module")
 def xf():
@@ -107,9 +105,8 @@ def make_plane_pair(img, K, rvec, t, out_hw=None):
     return warped, T
 
 
-def test_batched_harness_equals_per_pair_and_reference_auc(xf, oracle_state, assets_vga):
-    from accelerated_features_b200.evalharness import batched_matcher, run_pose_benchmark
-    ref_img, tgt_img = assets_vga
+def plane_pose_samples(ref_img, tgt_img):
+    """Four synthetic two-view samples of the asset images (two image shapes) in run_pose_benchmark's format."""
     K = np.array([[520.0, 0, 320], [0, 520.0, 240], [0, 0, 1]])
     samples = []
     poses = [((0.02, -0.05, 0.03), (0.10, 0.02, 0.05)), ((-0.04, 0.06, -0.05), (-0.08, 0.05, 0.10)),
@@ -124,6 +121,12 @@ def test_batched_harness_equals_per_pair_and_reference_auc(xf, oracle_state, ass
         warped, T = make_plane_pair(base, Kc, rv, np.asarray(t))
         samples.append({"image0": base, "image1": warped, "scale0": np.ones(2, np.float32), "scale1": np.ones(2, np.float32),
                         "K0": Kc, "K1": Kc, "T_0to1": T})
+    return samples
+
+
+def test_batched_harness_equals_per_pair_and_reference_auc(xf, golden, assets_vga):
+    from accelerated_features_b200.evalharness import batched_matcher, run_pose_benchmark
+    samples = plane_pose_samples(*assets_vga)
     match_pairs = batched_matcher(xf, "sparse", top_k=2048, batch_size=3)
     pairs = [(s["image0"], s["image1"]) for s in samples]
     got = match_pairs(pairs)
@@ -131,21 +134,10 @@ def test_batched_harness_equals_per_pair_and_reference_auc(xf, oracle_state, ass
         s0, s1 = xf.match_xfeat(a, b, top_k=2048)
         assert np.array_equal(g0, s0) and np.array_equal(g1, s1)
 
-    # the reference pipeline: unmodified modules.xfeat.XFeat on the CPU, one pair at a time (oracle/_ref), else the oracle port
-    from oracle import build_ref
-    if build_ref.available():
-        from accelerated_features_b200 import weights as _w
-        sd = {k: torch.as_tensor(v) for k, v in _w.load_state_dict(_w.DEFAULT_WEIGHTS).items()}
-        real = torch.cuda.is_available
-        torch.cuda.is_available = lambda: False                     # the reference picks CUDA when it sees one (xfeat.py:25)
-        try:
-            ref_xf = build_ref.import_reference()(weights=sd, top_k=2048)
-        finally:
-            torch.cuda.is_available = real
-        ref_matcher = lambda ps: [ref_xf.match_xfeat(a, b, top_k=2048) for a, b in ps]        # noqa: E731
-    else:
-        ref_matcher = lambda ps: [orc.match_xfeat(oracle_state, a, b, 2048) for a, b in ps]   # noqa: E731
-    want = ref_matcher(pairs)
+    # the reference pipeline: the unmodified modules.xfeat.XFeat's match_xfeat on the CPU, one pair at a time, stored by
+    # tools/make_golden_pose.py
+    g = golden("g6_pose_matches.npz")
+    want = [(g[f"mkpts0_{i}"], g[f"mkpts1_{i}"]) for i in range(len(samples))]
     for (g0, g1), (w0, w1) in zip(got, want):
         gs = {tuple(map(float, np.concatenate([a, b]))) for a, b in zip(g0, g1)}
         ws = {tuple(map(float, np.concatenate([a, b]))) for a, b in zip(w0, w1)}
@@ -157,7 +149,7 @@ def test_batched_harness_equals_per_pair_and_reference_auc(xf, oracle_state, ass
         return estimate_pose_opencv(*a, **k)
 
     mine = run_pose_benchmark(match_pairs, samples, ransac_thr=2.5, batch_size=3, pose_fn=pose_fn)
-    theirs = run_pose_benchmark(ref_matcher, samples, ransac_thr=2.5, batch_size=1, pose_fn=pose_fn)
+    theirs = run_pose_benchmark(lambda ps: want, samples, ransac_thr=2.5, batch_size=len(samples), pose_fn=pose_fn)
     print("AUC batched B200:", {k: round(v, 4) for k, v in mine.items() if k != "pairs"})
     print("AUC reference   :", {k: round(v, 4) for k, v in theirs.items() if k != "pairs"})
     from tests.parity_util import record
