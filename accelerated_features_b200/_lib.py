@@ -26,6 +26,8 @@ SIGNATURES = {
     "xfeat_set_conv_impl": (None, [c_i]),
     "xfeat_set_halo_desc_mode": (None, [c_i]),
     "xfeat_get_conv_impl": (c_i, []),
+    "xfeat_set_block1_fused": (None, [c_i]),
+    "xfeat_get_block1_fused": (c_i, []),
     "xfeat_net_workspace_bytes": (c_sz, [c_i, c_i, c_i]),
     "xfeat_net": (c_i, [c_p, c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_sz, c_p]),
     "xfeat_sparse_workspace_bytes": (c_sz, [c_i, c_i, c_i, c_i]),
@@ -56,6 +58,7 @@ SIGNATURES = {
     "xfeat_ransac_essential": (c_i, [c_p, c_p, c_p, c_i, c_i, c_f, c_i, C.c_uint32, c_p, c_p, c_p, c_p, c_sz, c_p]),
     "xfeat_debug_conv_layer": (c_i, [c_p, c_i, c_p, c_i, c_i, c_i, c_p, c_p]),
     "xfeat_debug_conv_layer_tc": (c_i, [c_p, c_i, c_p, c_i, c_i, c_i, c_p, c_p, c_sz, c_p]),
+    "xfeat_debug_block1_tail": (c_i, [c_p, c_p, c_p, c_i, c_i, c_i, c_p, c_p, c_sz, c_p]),
 }
 
 

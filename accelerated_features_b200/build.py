@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libxfeat_sm100.so")
 OBJ = os.path.join(HERE, "build")
-SOURCES = ["api.cu", "prep.cu", "stem.cu", "conv_simt.cu", "conv_tc.cu", "conv_tc_halo.cu", "head_chain_tc.cu", "heads.cu", "sparse.cu", "dense.cu", "mnn.cu", "mnn_tc.cu", "mnn_fast.cu", "refine.cu", "mlp_tc.cu", "helpers.cu", "ransac.cu"]
+SOURCES = ["api.cu", "prep.cu", "stem.cu", "conv_simt.cu", "conv_tc.cu", "conv_tc_halo.cu", "block1_tc.cu", "head_chain_tc.cu", "heads.cu", "sparse.cu", "dense.cu", "mnn.cu", "mnn_tc.cu", "mnn_fast.cu", "refine.cu", "mlp_tc.cu", "helpers.cu", "ransac.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "--expt-relaxed-constexpr",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "-Xptxas", "-v"]
 

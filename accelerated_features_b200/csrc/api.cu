@@ -173,11 +173,10 @@ extern "C" int xfeat_net(xfeat_ctx* ctx, const float* d_xn, int B, int H, int W,
     __half *s4a = (__half*)ws.x1s, *s4b = (__half*)ws.t4a, *s4c = (__half*)ws.x2;
     __half *s8a = (__half*)ws.t8a, *s8b = (__half*)ws.t8b, *s16a = (__half*)ws.t16a, *s16b = (__half*)ws.t16b;
     if (g_conv_impl == 2) {
-      // block1.0/1.1 on CUDA cores (K = 9 / 36), block1.2 (halo) and block1.3 + skip1 (stride 2) on tcgen05 with 32-byte
-      // operand rows [hi(8)|lo(8)]                                                 model.py:43-48,139-140
+      // block1.0/1.1 on CUDA cores (K = 9 / 36), block1.2 and block1.3 + skip1 (stride 2) in one tcgen05 kernel with 32-byte
+      // operand rows [hi(8)|lo(8)] (block1_tc.cu)                                  model.py:43-48,139-140
       XF_RUN(launch_stem_chain(ctx->h_weights, ctx->table, d_xn, ws.a1, ws.a2, ws.a3, nullptr, nullptr, B, H, W, st, 1));
-      XF_RUN(launch_conv_tc(ctx, L_B1_2, (const __half*)ws.a2, B, H / 2, W / 2, (__half*)ws.a3, nullptr, st));
-      XF_RUN(launch_conv_tc(ctx, L_B1_3, (const __half*)ws.a3, B, H / 2, W / 2, s4a, nullptr, st, d_xn));
+      XF_RUN(launch_block1_tail(ctx, (const __half*)ws.a2, d_xn, B, H4, W4, (__half*)ws.a3, s4a, nullptr, st));
     } else {
       XF_RUN(launch_stem_chain(ctx->h_weights, ctx->table, d_xn, ws.a1, ws.a2, ws.a3, nullptr, s4a, B, H, W, st));
     }

@@ -187,6 +187,8 @@ int launch_fine_mlp_tc(const xfeat_ctx* ctx, const __half* X_split, int rows_cap
                        float* logits, cudaStream_t st);
 int launch_conv_tc(const xfeat_ctx* ctx, int layer, const __half* in_split, int B, int H, int W, __half* out_split,
                    float* out_f32, cudaStream_t st, const float* skip_xn = nullptr);
+int launch_block1_tail(const xfeat_ctx* ctx, const __half* a2_split, const float* xn, int B, int H4, int W4, __half* a3_split,
+                       __half* out_split, float* out_f32, cudaStream_t st);
 int launch_head_chain(const xfeat_ctx* ctx, int mode, const void* in, int B, int Hc, int Wc, float* out, float* logits,
                       cudaStream_t st);
 int launch_split_nhwc(const float* in, __half* out, int64_t npix, int C, int CP, cudaStream_t st);

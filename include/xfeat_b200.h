@@ -99,6 +99,11 @@ XF_API int xfeat_preprocess_scaled(const void* d_img, int dtype, int B, int C, i
 XF_API void xfeat_set_halo_desc_mode(int mode);
 XF_API void xfeat_set_conv_impl(int impl);
 XF_API int xfeat_get_conv_impl(void);
+/* block1.2 -> block1.3 + skip1 of conv impl 2 (process-wide): 1 (default) = one fused tcgen05 kernel that keeps the
+ * half-resolution activation in shared memory, 0 = the two-kernel path.  XFEAT_BLOCK1_UNFUSED=1 in the environment forces 0;
+ * xfeat_get_block1_fused reports the path in effect.  Both paths give bit-identical results. */
+XF_API void xfeat_set_block1_fused(int on);
+XF_API int xfeat_get_block1_fused(void);
 XF_API size_t xfeat_net_workspace_bytes(int B, int H, int W);
 /* replaces: XFeatModel.forward (model.py:123-154) minus the normalisation (done by xfeat_preprocess), plus
  * get_kpts_heatmap (xfeat.py:242-247) fused after keypoint_head.
@@ -267,6 +272,12 @@ XF_API int xfeat_debug_conv_layer(xfeat_ctx* ctx, int layer, const float* d_in, 
 /* Test hook: one 64->64 stride-1 layer through the tensor-core kernel, fp32 NHWC in/out; d_scratch >= B*H*W*256 bytes. */
 XF_API int xfeat_debug_conv_layer_tc(xfeat_ctx* ctx, int layer, const float* d_in, int B, int H, int W, float* d_out,
                                      void* d_scratch, size_t scratch_bytes, void* stream);
+
+/* Test hook: block1.2 -> block1.3 + skip1 on the tensor cores (the path xfeat_set_block1_fused selects).  d_a2
+ * (B,H/2,W/2,8) fp32 NHWC block1.1 output, d_xn (B,H,W) -> d_x1s (B,H/4,W/4,24) = block1(x) + skip1(x); H, W multiples of 4;
+ * d_scratch >= B*(H/2)*(W/2)*64 bytes. */
+XF_API int xfeat_debug_block1_tail(xfeat_ctx* ctx, const float* d_a2, const float* d_xn, int B, int H, int W, float* d_x1s,
+                                   void* d_scratch, size_t scratch_bytes, void* stream);
 
 #ifdef __cplusplus
 }
